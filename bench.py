@@ -4,6 +4,7 @@ fraction of the HBM-read roofline).
 
     python bench.py --gpus N --steps K --warmup W [--config C2|C3|C4|C5]    # this repo's sm_100a path
     python bench.py --impl reference --gpus N --steps K ... [--config ..]   # the CPU restatement on the host cores
+    python bench.py ... --dump-outputs DIR     # also write what the last timed step computed, DIR/<name>.npy (float64)
 
 Configs (BASELINE.json `configs`, SURVEY.md section 8d; the default and the headline is C2):
   C2  100 000 synthetic files x 4 KiB per GPU (weak scaling), tokenise + line-hash + classify + aggregate
@@ -33,6 +34,7 @@ sys.path.insert(0, os.path.join(ROOT, "tosem-2021-replication_b200"))
 
 import numpy as np  # noqa: E402
 
+sys.dont_write_bytecode = True         # the benchmark leaves the tree as the build left it (it may be read-only)
 FILE_SIZE = 4096
 N_GROUPS = 9
 MAX_BATCH_FILES_4K = 500000            # 500 000 x 4 KiB = 2.048e9 B: the largest 4 KiB batch an int32-indexed arena holds
@@ -60,7 +62,30 @@ def parse():
     ap.add_argument("--scale", type=float, default=1.0, help="shrink the workload (smoke runs); 1.0 = the named config")
     ap.add_argument("--e2e-steps", type=int, default=0, help="0 = min(steps, 10)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the outputs of the last timed step to DIR/<name>.npy (float64)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 path")
+    return args
+
+
+DUMP_MAX_ROWS = 800000                 # per-file / per-pair rows --dump-outputs keeps: <= 8 float64 columns, < 52 MB
+
+
+def dump_outputs(out_dir, rows, tables):
+    """--dump-outputs: every array as out_dir/<name>.npy in float64, which holds these integers exactly (64-bit digests
+    come split into 32-bit halves).  rows: per-file or per-pair columns; past DUMP_MAX_ROWS rows a fixed seeded sample of
+    them, whose row numbers go to row_index.npy.  tables: arrays written whole."""
+    os.makedirs(out_dir, exist_ok=True)
+    n = len(next(iter(rows.values())))
+    if n > DUMP_MAX_ROWS:
+        keep = np.sort(np.random.default_rng(0).choice(n, DUMP_MAX_ROWS, replace=False))
+        rows = dict({k: v[keep] for k, v in rows.items()}, row_index=keep)
+    for name, a in list(rows.items()) + list(tables.items()):
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a).astype(np.float64))
 
 
 def config_json(args, n, extra):
@@ -385,6 +410,14 @@ def bench_scan(args, ts, torch, env):
         mine = torch.tensor([glob_assert], dtype=torch.int64, device="cuda")
         dist.all_reduce(mine)
         assert int(stage[k][N_GROUPS * 128:(N_GROUPS + 1) * 128].sum().item()) == int(mine.item()), "allreduced counts"
+    if args.dump_outputs and rank == 0:                     # this rank's files in batch order, its tables summed over batches
+        st = np.concatenate([r["stats"] for r in res])
+        tables = {k: sum(r[k] for r in res) for k in ("group_counts", "global_counts", "totals")}
+        if n > 1:
+            tables["counts_all_ranks"] = stage[(it[0] - 1) & 1].cpu().numpy()
+        dump_outputs(args.dump_outputs, {"n_lines": st["n_lines"], "n_assert": st["n_assert"], "n_headers": st["n_headers"],
+                                         "n_fixture": st["n_fixture"], "digest_lo": st["digest"] & np.uint64(0xFFFFFFFF),
+                                         "digest_hi": st["digest"] >> np.uint64(32)}, tables)
     # ---- e2e through the host C-ABI path
     ke = args.e2e_steps or min(args.steps, 10)
     nf_rank = sum(c.n_files for c in batches)
@@ -517,6 +550,9 @@ def bench_diff(args, ts, torch, env):
     lb = sc.line_hashes(b)[0]
     assert np.array_equal(add - rem, np.diff(lb) - np.diff(la)), "added - removed must equal the change in line count"
     assert int(add.sum() + rem.sum()) > 0
+    if args.dump_outputs and rank == 0:                     # this rank's pairs in ascending logical order
+        dump_outputs(args.dump_outputs, dict({"added": add, "removed": rem}, **{f: det[f] for f in det.dtype.names}),
+                     {"churn_totals_all_ranks": tot.cpu().numpy()} if n > 1 else {})
     ke = args.e2e_steps or min(args.steps, 10)
 
     def e2e_step():

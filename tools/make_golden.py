@@ -552,9 +552,10 @@ def _is_utf8(b):
         return False
 
 
-def c1_summary(ledger, write=True):
-    """Config C1: the oracle over the bundled corpus (test files with a scannable extension)."""
-    projects, files, ext, grp, names = c1_collect()
+def c1_summary(ledger, write=True, corpus=None):
+    """Config C1: the oracle over the bundled corpus (test files with a scannable extension).  corpus = (projects,
+    files, ext, grp) of those files from elsewhere: the tests pass tests/golden/c1_testfiles.npz."""
+    projects, files, ext, grp = corpus or c1_collect()[:4]
     arena, off, length = orc.pack(files)
     res = orc.scan(arena, off, length, np.array(ext, np.uint8), np.array(grp, np.uint16), len(projects), events=False)
     st = res["stats"]
